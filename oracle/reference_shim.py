@@ -88,3 +88,26 @@ def load_reference_model(cfg, state_dict: Dict[str, torch.Tensor]):
 
 def tokens_from_text(text: str) -> List[int]:
     return [int(t) for t in text.split()]
+
+
+def tensor_sha256(*tensors: torch.Tensor) -> str:
+    """sha256 of the raw bytes of the tensors, in order (bit-identity against a stored reference result)"""
+    import hashlib
+
+    h = hashlib.sha256()
+    for t in tensors:
+        h.update(t.detach().contiguous().reshape(-1).view(torch.uint8).numpy().tobytes())
+    return h.hexdigest()
+
+
+def host_arithmetic() -> Dict[str, str]:
+    """What decides the bits of the oracle's CPU bf16 results on this host: ATen's vector ISA and the oneDNN kernels
+    behind bf16 linear / attention (AMX tiles, AVX-512 bf16, ...), probed on seeded inputs.  The stored reference
+    results can only be matched bit for bit on a host where this is the same as on the host that recorded them."""
+    import torch.nn.functional as F
+
+    g = torch.Generator().manual_seed(0)
+    x, w = (torch.randn(64, 1152, generator=g).to(torch.bfloat16), torch.randn(1152, 1152, generator=g).to(torch.bfloat16))
+    q, k, v = (torch.randn(1, 4, 96, 64, generator=g).to(torch.bfloat16) for _ in range(3))
+    return {"cpu_capability": torch.backends.cpu.get_cpu_capability(),
+            "bf16_probe_sha256": tensor_sha256(F.linear(x, w), F.scaled_dot_product_attention(q, k, v))}

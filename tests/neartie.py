@@ -42,6 +42,23 @@ def check_objects(got_bins, want_bins, want_ulps, what=""):
     return len(want_bins)
 
 
+def reference_bitwise(exact_bf16: bool = False) -> dict:
+    """tests/golden/reference_bitwise.json (oracle/make_golden_bitwise.py): what the unmodified reference computed.
+    `exact_bf16`: the caller compares CPU bf16 results bit for bit, which only a host with the recording host's CPU
+    arithmetic can reproduce (see above); elsewhere the test is skipped and the fixture replays stand in for it."""
+    import json
+    import os
+
+    import pytest
+
+    from oracle import reference_shim as R
+
+    gold = json.load(open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_bitwise.json")))
+    if exact_bf16 and R.host_arithmetic() != gold["host"]:
+        pytest.skip(f"this host's CPU bf16 arithmetic {R.host_arithmetic()} is not the recording host's {gold['host']}")
+    return gold
+
+
 def json_close(got, want, float_tol, path=""):
     """structural equality of two JSON values: ints / strings / bools / shapes exact, floats within
     float_tol(path) where path is the key path with list indices dropped.  Returns a list of mismatches."""

@@ -5,6 +5,7 @@ import os
 import subprocess
 import sys
 
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
@@ -112,3 +113,24 @@ def test_parity_gate_accepts_near_tie_flips_and_rejects_clear_mismatches(monkeyp
     # 4. free-running happens to agree but a teacher-forced step disagrees at a clear margin: fails too
     rep, _ = _gate(monkeypatch, pad(base), pad(forced), base, wide)
     assert not rep["ok"] and "teacher-forced" in rep["error"]
+
+
+def test_dump_outputs_writes_the_token_ids_as_float32(tmp_path):
+    import numpy as np
+    import torch
+
+    import bench
+
+    tokens = torch.tensor([[1, 51199, 0], [7, 8, 9]], dtype=torch.int32)
+    bench.dump_outputs(str(tmp_path / "out"), tokens)
+    got = np.load(tmp_path / "out" / "tokens.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, tokens.numpy())
+
+
+@pytest.mark.parametrize("argv,flag", [(["--steps", "0"], "--steps"),
+                                       (["--impl", "reference", "--dump-outputs", "out"], "--dump-outputs")])
+def test_arguments_bench_cannot_honour_are_rejected(tmp_path, argv, flag):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + argv, capture_output=True, text=True,
+                       cwd=tmp_path, timeout=300)
+    assert r.returncode == 2 and flag in r.stderr and r.stdout.strip() == ""
+    assert not (tmp_path / "out").exists()

@@ -9,6 +9,7 @@ import torch
 from moondream_b200 import config as C, synth
 from moondream_b200 import weights as W
 from moondream_b200.engine import prepare_weights
+from oracle.make_golden_bitwise import legacy_dict as _legacy_dict
 
 
 def test_config_defaults_match_reference_values():
@@ -23,22 +24,16 @@ def test_config_defaults_match_reference_values():
 
 
 def test_config_dict_equals_the_reference_config_dict():
-    """Build container only: `MoondreamConfig().to_dict()` (config.py:75-94) key for key, and a dict produced by the
-    reference's config loads into ours (the `from_dict` a maintainer would feed with the reference's config JSONs)."""
-    from oracle import reference_shim as R
+    """`MoondreamConfig().to_dict()` (config.py:75-94) key for key against the unmodified reference's
+    (tests/golden/reference_bitwise.json), and a dict produced by the reference's config loads into ours (the
+    `from_dict` a maintainer would feed with the reference's config JSONs)."""
+    from neartie import reference_bitwise
 
-    if not R.reference_available():
-        pytest.skip("/root/reference is not present on this box")
-    import sys
-
-    sys.path.insert(0, R.REFERENCE_ROOT)
-    from moondream.torch.config import MoondreamConfig as RefConfig
-
-    ref = RefConfig().to_dict()
-    assert C.MoondreamConfig().to_dict() == ref
-    assert C.MoondreamConfig.from_dict(json.loads(json.dumps(ref))) == C.MoondreamConfig()
-    small = C.moondream_0_5b().to_dict()
-    assert RefConfig.from_dict(small).to_dict() == small
+    gold = reference_bitwise()["config"]
+    assert C.MoondreamConfig().to_dict() == gold["default"]
+    assert C.MoondreamConfig.from_dict(json.loads(json.dumps(gold["default"]))) == C.MoondreamConfig()
+    small = json.loads(json.dumps(C.moondream_0_5b().to_dict()))
+    assert gold["moondream_0_5b_round_trip"] == small
 
 
 def test_config_dict_round_trip_and_partial_dict():
@@ -58,14 +53,6 @@ def test_validate_rejects_what_the_kernels_do_not_implement():
         C.MoondreamConfig(text=C.TextConfig(group_size=64)).validate()       # the reference hard-codes 128
     with pytest.raises(ValueError):
         C.preset("no-such-model")
-
-
-def _legacy_dict(cfg, sd):
-    inv = {v: k for k, v in W.legacy_key_map(cfg).items()}
-    out = {inv[k]: v for k, v in sd.items() if k in inv}
-    out["region_model.coordinate_features.weight"] = sd["region.coord_features"].T.contiguous()
-    out["region_model.size_features.weight"] = sd["region.size_features"].T.contiguous()
-    return out
 
 
 @pytest.mark.parametrize("layout", ["canonical", "model_prefixed", "legacy", "legacy_orig_mod"])
@@ -127,44 +114,26 @@ def test_prepare_weights_pads_for_tma_without_changing_values():
 @pytest.mark.parametrize("layout,fmt", [("legacy", "safetensors"), ("legacy_orig_mod", "pt"), ("model_prefixed", "safetensors"),
                                         ("canonical", "pt")])
 def test_loader_agrees_with_the_reference_loader(tmp_path, layout, fmt):
-    """Build container only: the same file goes through the unmodified reference's `load_weights_into_model`
-    (weights.py:120-171) into the reference model and through ours; every parameter must come out identical, which pins
-    the legacy key map (and the transposed region feature tensors) to the reference rather than to this repo's reading of it."""
-    from oracle import reference_shim as R
+    """The same file went through the unmodified reference's `load_weights_into_model` (weights.py:120-171) into the
+    reference model and goes through ours; every parameter must come out identical, which pins the legacy key map (and
+    the transposed region feature tensors) to the reference rather than to this repo's reading of it.
+    tests/golden/reference_bitwise.json holds what the reference was fed (names, dtypes, shapes and bytes of the file,
+    so the file written here must be that file) and the parameters it ended with."""
+    from neartie import reference_bitwise
 
-    if not R.reference_available():
-        pytest.skip("/root/reference is not present on this box")
-    import sys
+    from oracle.make_golden_bitwise import checkpoint_sha256, weight_file
+    from oracle.reference_shim import tensor_sha256
 
-    from safetensors.torch import save_file
-
+    gold = reference_bitwise()["loader"]
     cfg = C.tiny()
     sd = synth.synthetic_state_dict(cfg, 2)
-    if layout == "canonical":
-        tensors = dict(sd)
-    elif layout == "model_prefixed":
-        tensors = {"model." + k: v for k, v in sd.items()}
-    else:
-        tensors = _legacy_dict(cfg, sd)
-        if layout == "legacy_orig_mod":
-            tensors = {k.replace("text_model.", "text_model._orig_mod.", 1): v for k, v in tensors.items()}
-    path = str(tmp_path / ("w." + ("safetensors" if fmt == "safetensors" else "pt")))
-    if fmt == "safetensors":
-        save_file({k: v.contiguous() for k, v in tensors.items()}, path)
-    else:
-        torch.save(tensors, path)
-
-    ref = R.load_reference_model(cfg, synth.synthetic_state_dict(cfg, 5))      # different weights: must be overwritten
-    sys.path.insert(0, R.REFERENCE_ROOT)
-    from moondream.torch.weights import load_weights_into_model as ref_load
-
-    ref_load(path, ref)
-    theirs = {k: v for k, v in ref.state_dict().items() if "kv_cache" not in k}
+    path = weight_file(tmp_path, cfg, sd, layout, fmt)
+    assert checkpoint_sha256(path) == gold["file_sha256"][f"{layout}-{fmt}"], "not the file the reference loader was fed"
     ours = W.load_state_dict_from_file(path, cfg)
-    assert set(ours) == set(sd)
+    assert sorted(ours) == sorted(sd) == gold["keys"]
+    assert tensor_sha256(*[ours[k] for k in gold["keys"]]) == gold["sha256"][f"{layout}-{fmt}"]
     for k in sd:
-        assert k in theirs, k
-        assert torch.equal(theirs[k], sd[k]) and torch.equal(ours[k], sd[k]), k
+        assert torch.equal(ours[k], sd[k]), k
 
 
 def test_native_safetensors_reader_matches_the_safetensors_package(tmp_path):
@@ -268,22 +237,19 @@ def test_native_safetensors_reader_rejects_malformed_and_hostile_headers(tmp_pat
 def test_variant_files_are_found_and_renamed_like_the_reference(tmp_path, monkeypatch):
     """settings["variant"] (row f4): MoondreamModel._lora looks a variant id up in the reference's cache layout
     (lora.py:11-29: $HF_HUB_CACHE/md_variants/<id>/final.pt, else $HF_HOME/hub/...) and applies the reference's key
-    renames (lora.py:64-76) to checkpoints saved with the trainer's names.  Compared with the unmodified reference's
-    `variant_state_dict` where /root/reference exists; the expected tree is also spelt out so the test holds anywhere."""
+    renames (lora.py:64-76) to checkpoints saved with the trainer's names.  Compared with what the unmodified
+    reference's `variant_state_dict` made of the same file; the expected tree is also spelt out."""
     import pytest
 
     from moondream_b200 import config as C, synth
     from moondream_b200.moondream import MoondreamModel
+    from neartie import reference_bitwise
     from oracle import reference_shim as R
+    from oracle.make_golden_bitwise import trainer_named_lora
 
     cfg = C.tiny()
     flat = synth.synthetic_lora(cfg, 8, 0)                       # canonical names: text.blocks.{i}.{attn.qkv, attn.proj, mlp.fc1, mlp.fc2}.{A, B}
-    trainer = {}
-    for k, t in flat.items():                                    # the names the trainer saves (what the renames undo)
-        k2 = (k.replace("text.blocks", "text_model.transformer.h").replace(".attn.qkv", ".mixer.Wqkv")
-               .replace(".attn.proj", ".mixer.out_proj"))
-        k2 = k2[:-2] + ".parametrizations.weight.0" + k2[-2:]
-        trainer[k2] = t
+    trainer = trainer_named_lora(flat)                           # the names the trainer saves (what the renames undo)
     assert "text_model.transformer.h.0.mixer.Wqkv.parametrizations.weight.0.A" in trainer
     hub = tmp_path / "hub_cache"
     (hub / "md_variants" / "v1").mkdir(parents=True)
@@ -307,23 +273,11 @@ def test_variant_files_are_found_and_renamed_like_the_reference(tmp_path, monkey
     monkeypatch.setenv("HF_HOME", str(home))
     assert model._lora({"variant": "v2"}) == ("variant", 2) and sorted(seen[1]) == sorted(flat)
     assert model._lora({"variant": str(hub / "md_variants" / "v1" / "final.pt")}) == ("variant", 3)   # a path works too
-    if R.reference_available():
-        import sys
+    # the unmodified reference's variant_state_dict("v2") on the same file (tests/golden/reference_bitwise.json)
+    def tree_sha256(tree):
+        return {k: tree_sha256(v) for k, v in tree.items()} if isinstance(tree, dict) else R.tensor_sha256(tree)
 
-        if R.REFERENCE_ROOT not in sys.path:
-            sys.path.insert(0, R.REFERENCE_ROOT)
-        from moondream.torch import lora as ref_lora
-
-        ref_lora.variant_state_dict.cache_clear()
-        tree = ref_lora.variant_state_dict("v2")                                    # $HF_HOME/hub/md_variants/v2/final.pt
-        mine = synth.nest_lora(seen[1])
-
-        def same(a, b):
-            if isinstance(a, dict):
-                return isinstance(b, dict) and a.keys() == b.keys() and all(same(a[k], b[k]) for k in a)
-            return torch.equal(a, b)
-
-        assert same(tree, mine)
+    assert tree_sha256(synth.nest_lora(seen[1])) == reference_bitwise()["variant_tree_sha256"]
 
 
 def test_lora_variant_table_and_shape_checks():

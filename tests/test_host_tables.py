@@ -1,7 +1,6 @@
 """Host-built tables the kernels consume: the 256-entry pixel LUT (reference vision.py:33-40) and the RoPE table
 (rope.py:6-17 as text.py:215-219 calls it).  Both must be bit-identical to what the reference computes."""
 import numpy as np
-import pytest
 import torch
 
 from moondream_b200 import config as C
@@ -26,16 +25,13 @@ def test_pixel_lut_is_the_reference_normalisation():
     assert torch.equal(crops[0], want)
 
 
-@pytest.mark.skipif(not R.reference_available(), reason="/root/reference only exists in the build container")
 def test_rope_table_is_the_reference_table():
-    import sys
+    """against precompute_freqs_cis of the unmodified reference (tests/golden/reference_bitwise.json)"""
+    from neartie import reference_bitwise
 
-    sys.path.insert(0, R.REFERENCE_ROOT)
-    from moondream.torch.rope import precompute_freqs_cis
-
-    for cfg in (C.tiny(), C.preset("moondream-2b")):
-        t = cfg.text
-        ref = precompute_freqs_cis(t.dim // (2 * t.n_heads), t.max_context)          # text.py:215-219
+    gold = reference_bitwise()["rope_sha256"]
+    for preset in ("tiny", "moondream-2b"):
+        t = C.preset(preset).text
         mine = rope_table(t.head_dim, t.max_context)
         assert mine.dtype == torch.float32 and tuple(mine.shape) == (t.max_context, t.head_dim // 4, 2)
-        assert ref.dtype == torch.float32 and torch.equal(mine, ref)
+        assert R.tensor_sha256(mine) == gold[preset], preset

@@ -68,34 +68,26 @@ def test_select_tiling_properties():
 
 
 def test_random_sizes_against_the_oracle_and_the_reference():
-    """Ragged sizes, extreme aspect ratios and every max_crops: product == oracle restatement bit for bit, and, in the
-    build container, == the unmodified reference (`image_crops.py:58-167`, PIL-Lanczos branch); margins other than the
-    default too.  Reconstruction of per-crop index maps must tile the stitched grid without holes."""
+    """Ragged sizes, extreme aspect ratios and every max_crops: product == oracle restatement bit for bit == the
+    unmodified reference (`image_crops.py:58-167`, PIL-Lanczos branch; tests/golden/reference_bitwise.json); margins
+    other than the default too.  Reconstruction of per-crop index maps must tile the stitched grid without holes."""
     from moondream_b200 import synth
-    from oracle import reference_shim as R
+    from neartie import reference_bitwise
+    from oracle.make_golden_bitwise import crop_cases
+    from oracle.reference_shim import tensor_sha256
     from oracle.moondream_oracle import overlap_crops
 
-    ref_crop = None
-    if R.reference_available():
-        import sys
-
-        sys.path.insert(0, R.REFERENCE_ROOT)
-        from moondream.torch.image_crops import overlap_crop_image as ref_crop
-    rng = np.random.default_rng(123)
-    sizes = [(1, 1), (1, 900), (900, 1), (377, 379), (379, 377), (266, 267), (1200, 90)]
-    sizes += [(int(rng.integers(2, 1100)), int(rng.integers(2, 1100))) for _ in range(14)]
-    for n, (h, w) in enumerate(sizes):
-        max_crops = int(rng.integers(1, 13))
-        margin = 4 if n % 3 else int(rng.integers(1, 7))
-        img = synth.synthetic_image(1000 + n, h, w)
+    gold = reference_bitwise()["crops"]
+    cases = crop_cases()
+    assert len(cases) == len(gold) == 21
+    for (idx, h, w, max_crops, margin), theirs in zip(cases, gold):
+        img = synth.synthetic_image(idx, h, w)
         out = overlap_crop_image(img, overlap_margin=margin, max_crops=max_crops)
         th, tw = out["tiling"]
         assert out["crops"].dtype == np.uint8 and out["crops"].shape == (1 + th * tw, 378, 378, 3) and th * tw <= max_crops
         mine, tiling = overlap_crops(img, margin, max_crops)
         assert tuple(tiling) == (th, tw) and np.array_equal(mine, out["crops"]), (h, w, max_crops, margin)
-        if ref_crop is not None:
-            theirs = ref_crop(img, overlap_margin=margin, max_crops=max_crops)
-            assert tuple(theirs["tiling"]) == (th, tw) and np.array_equal(theirs["crops"], out["crops"]), (h, w)
+        assert theirs["tiling"] == [th, tw] and theirs["sha256"] == tensor_sha256(torch.from_numpy(out["crops"])), (h, w)
         # stitching per-crop constant maps: every output cell is owned by exactly one crop (no holes, no NaNs)
         grid = 27
         feats = [torch.full((grid, grid, 1), float(i)) for i in range(th * tw)]

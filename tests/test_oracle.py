@@ -1,5 +1,5 @@
-"""The oracle (CPU restatement of the reference) against (a) the committed golden fixtures produced by
-the unmodified reference and (b) the reference itself when /root/reference is present (build container)."""
+"""The oracle (CPU restatement of the reference) against the committed golden fixtures produced by the unmodified
+reference: replays with the near-tie rule (tests/neartie.py), and bit for bit against reference_bitwise.json."""
 import json
 import os
 
@@ -75,104 +75,78 @@ def test_fp32_truth_is_close_to_bf16_port(tiny):
     assert ((a - b).norm() / b.norm()).item() < 5e-2
 
 
-@pytest.mark.skipif(not R.reference_available(), reason="/root/reference only exists in the build container")
 def test_oracle_is_bit_identical_to_reference(tiny):
-    from PIL import Image
+    """encode_image + caption("short") of the unmodified reference (tests/golden/reference_bitwise.json): every layer's
+    KV cache bit for bit and the greedy tokens"""
+    from neartie import reference_bitwise
 
     cfg, sd, orc = tiny
-    ref = R.load_reference_model(cfg, sd)
-    img = synth.synthetic_image(11, 600, 450)
-    with torch.inference_mode():
-        enc = ref.encode_image(Image.fromarray(img))
-    o_enc = orc.encode_image(img)
-    for (k, v), (ok, ov) in zip(enc.caches, o_enc.caches):
-        assert torch.equal(k, ok) and torch.equal(v, ov)
-    text = ref.caption(enc, "short", settings={"temperature": 0, "max_tokens": 10})["caption"]
+    gold = reference_bitwise(exact_bf16=True)["tiny_caption"]
+    o_enc = orc.encode_image(synth.synthetic_image(*gold["image"]))
+    assert len(o_enc.caches) == cfg.text.n_layers
+    assert R.tensor_sha256(*[t for kv in o_enc.caches for t in kv]) == gold["kv_sha256"]
     gen = orc.generate(o_enc, cfg.tokenizer.templates["caption"]["short"], 10)
-    assert R.tokens_from_text(text) == gen.tokens
+    assert gen.tokens == gold["tokens"]
 
 
-@pytest.mark.skipif(not R.reference_available(), reason="/root/reference only exists in the build container")
 def test_oracle_spatial_refs_and_sampling_are_bit_identical_to_reference(tiny):
     """query(spatial_refs=...) (moondream.py:293-301, region.py:96-136): logits and hidden states of the prompt prefill
     with point and box references, then the greedy tokens; and seeded nucleus sampling (moondream.py:270-278)."""
-    from PIL import Image
+    from neartie import reference_bitwise
 
     cfg, sd, orc = tiny
     tk = cfg.tokenizer
-    ref = R.load_reference_model(cfg, sd)
-    img = synth.synthetic_image(2, 500, 700)
-    with torch.inference_mode():
-        enc = ref.encode_image(Image.fromarray(img))
-    o_enc = orc.encode_image(img)
-    seen = []
-    orig = ref._prefill_prompt
-
-    def recording(prompt_tokens, pos, *a, **k):
-        out = orig(prompt_tokens, pos, *a, **k)
-        seen.append((prompt_tokens.flatten().tolist(), out[0].clone(), out[1].clone()))
-        return out
-
-    ref._prefill_prompt = recording
-    try:
-        for refs in ([(0.25, 0.75)], [(0.1, 0.2, 0.5, 0.9)], [(0.25, 0.75), (0.1, 0.2, 0.5, 0.9), (0.6, 0.6)]):
-            seen.clear()
-            text = ref.query(enc, "15 16", spatial_refs=refs, settings={"temperature": 0, "max_tokens": 8})["answer"]
-            prompt, ref_logits, ref_hidden = seen[0]
-            assert prompt.count(tk.coord_id) == 2 * len(refs) and prompt.count(tk.size_id) == sum(len(r) == 4 for r in refs)
-            orc.load_encoded(o_enc)
-            logits, hidden, _, _ = orc.prefill_prompt(prompt, o_enc.pos, orc.spatial_prompt_embeds(prompt, refs))
-            assert torch.equal(logits, ref_logits) and torch.equal(hidden, ref_hidden)
-            plain = orc.prefill_prompt(prompt, o_enc.pos)[0]
-            assert not torch.equal(plain, ref_logits)                      # the references really enter the prompt
-            assert orc.generate(o_enc, prompt, 8, spatial_refs=refs).tokens == R.tokens_from_text(text)
-    finally:
-        ref._prefill_prompt = orig
-    prompt = synth.synthetic_prompt(3, 6, cfg.text.vocab_size)
-    for seed, temp, top_p in ((5, 0.5, 0.3), (6, 1.5, 0.9)):
-        ref.load_encoded_image(enc)
-        torch.manual_seed(seed)
-        text = "".join(ref._generate_answer(torch.tensor([prompt]), enc.pos,
-                                            {"temperature": temp, "top_p": top_p, "max_tokens": 10}))
-        torch.manual_seed(seed)
-        assert orc.generate(o_enc, prompt, 10, temperature=temp, top_p=top_p).tokens == R.tokens_from_text(text)
+    gold = reference_bitwise(exact_bf16=True)
+    o_enc = orc.encode_image(synth.synthetic_image(*gold["tiny_spatial_refs"]["image"]))
+    for c in gold["tiny_spatial_refs"]["cases"]:
+        refs = [tuple(r) for r in c["spatial_refs"]]
+        prompt = c["prompt"]
+        assert prompt.count(tk.coord_id) == 2 * len(refs) and prompt.count(tk.size_id) == sum(len(r) == 4 for r in refs)
+        orc.load_encoded(o_enc)
+        logits, hidden, _, _ = orc.prefill_prompt(prompt, o_enc.pos, orc.spatial_prompt_embeds(prompt, refs))
+        assert R.tensor_sha256(logits) == c["logits_sha256"] and R.tensor_sha256(hidden) == c["hidden_sha256"]
+        plain = orc.prefill_prompt(prompt, o_enc.pos)[0]
+        assert not torch.equal(plain, logits)                          # the references really enter the prompt
+        assert orc.generate(o_enc, prompt, 8, spatial_refs=refs).tokens == c["tokens"]
+    sampling = gold["tiny_sampling"]
+    assert sampling["image"] == gold["tiny_spatial_refs"]["image"]
+    for c in sampling["cases"]:
+        torch.manual_seed(c["seed"])
+        got = orc.generate(o_enc, sampling["prompt"], 10, temperature=c["temperature"], top_p=c["top_p"]).tokens
+        assert got == c["tokens"], c
 
 
-@pytest.mark.skipif(not R.reference_available(), reason="/root/reference only exists in the build container")
 @pytest.mark.parametrize("preset,head_peak", [("moondream-2b", 3.0), ("moondream-0.5b", 0.0)])
 def test_oracle_is_bit_identical_to_reference_on_the_real_architectures(preset, head_peak):
     """The pin on the configurations BASELINE.json quotes, not only on the tiny presets.  Moondream-2B (text 2048 x 24
     layers x 32 heads, ViT 1152 x 27 layers with head_dim 72, vocab 51200) with the bench's synthetic weights (head
     peak 3), its image 0 / prompt 0; and Moondream-0.5B (text 1024 x 16 heads, ViT 720 x 10 heads, MLP width 2690).
-    The UNMODIFIED reference and the oracle must agree bit for bit on every layer of the 730-token KV prefix, on the
-    greedy tokens and on a 2-object detect.  (~80 s + ~25 s on 8 cores: two copies of each model.)"""
-    from PIL import Image
+    The oracle must reproduce what the UNMODIFIED reference computed (tests/golden/reference_bitwise.json) bit for bit
+    on every layer of the 730-token KV prefix, on the greedy tokens and on a 2-object detect."""
+    from neartie import reference_bitwise
 
+    gold = reference_bitwise(exact_bf16=True)["real_architectures"][preset]
+    assert gold["head_peak"] == head_peak
     cfg = C.preset(preset)
     sd = synth.synthetic_state_dict(cfg, 0, head_peak=head_peak)          # bench.py: HEAD_PEAK = 3 for the 2B
-    ref = R.load_reference_model(cfg, sd)
     orc = OracleModel(cfg, sd)
-    img = synth.synthetic_image(0, 378, 378)
-    with torch.inference_mode():
-        enc = ref.encode_image(Image.fromarray(img))
-    o_enc = orc.encode_image(img)
-    assert enc.pos == o_enc.pos == 730 and len(enc.caches) == cfg.text.n_layers
-    for (k, v), (ok, ov) in zip(enc.caches, o_enc.caches):
-        assert tuple(k.shape) == (1, cfg.text.n_kv_heads, 730, 64) and torch.equal(k, ok) and torch.equal(v, ov)
+    o_enc = orc.encode_image(synth.synthetic_image(0, 378, 378))
+    assert gold["pos"] == o_enc.pos == 730 and len(o_enc.caches) == cfg.text.n_layers
+    assert gold["kv_shape"] == [1, cfg.text.n_kv_heads, 730, 64]
+    assert all(tuple(t.shape) == tuple(gold["kv_shape"]) for kv in o_enc.caches for t in kv)
+    assert R.tensor_sha256(*[t for kv in o_enc.caches for t in kv]) == gold["kv_sha256"]
     prompt = synth.synthetic_prompt(0, 32, cfg.text.vocab_size)     # bench.py: PROMPT_LEN
-    ref.load_encoded_image(enc)
-    text = "".join(ref._generate_answer(torch.tensor([prompt]), enc.pos, {"temperature": 0, "max_tokens": 5}))
     gen = orc.generate(o_enc, prompt, 5)
-    assert R.tokens_from_text(text) == gen.tokens
+    assert gen.tokens == gold["tokens"]
     # the same five tokens open image 0's caption in every GPU bench run of the round (profiles/r02_bench_final.json:
-    # comparators.*.first_tokens, produced by the oracle's arithmetic on the B200) -- on hosts whose oneDNN path matches
+    # comparators.*.first_tokens, produced by the oracle's arithmetic on the B200)
     if preset == "moondream-2b" and gen.tokens != [1094, 22849, 11037, 121, 36410]:
         assert min(gen.margin_ulps) < 4.5, gen.tokens
     # region head at full width (detect: coordinate + size decode / encode interleaved with decoder steps, moondream.py:653-733)
     tk = cfg.tokenizer
-    det = ref.detect(enc, "17 23", settings={"max_objects": 2})["objects"]
     dprompt = tk.templates["detect"]["prefix"] + [17, 23] + tk.templates["detect"]["suffix"]
     o_det = orc.generate_points(o_enc, dprompt, True, 2)
+    det = gold["detect"]
     assert len(o_det) == len(det) and [{k: o[k] for k in d} for o, d in zip(o_det, det)] == det
 
 

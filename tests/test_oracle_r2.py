@@ -114,19 +114,21 @@ def test_apply_top_p_matches_the_reference():
         assert kept[0, nz].float().tolist() == c["kept_probs"]
 
 
-def test_round2_restatements_are_bit_identical_to_the_reference_here(tmp_path):
-    """runs only where /root/reference exists (the build container).  Regenerating the fixtures (into a scratch directory)
-    asserts oracle == reference bit for bit on every case, on THIS host; the regenerated files must then agree with the
-    committed ones: every integer / string exactly (tokens, bins, coordinates, texts), recorded margins and probes within
-    the host-to-host accumulation-order spread (tests/neartie.py)."""
-    from neartie import MARGIN_ULPS_TOL, json_close
+def test_round2_restatements_are_bit_identical_to_the_reference_here(tiny):
+    """Every case of oracle/make_golden_r2.py through the oracle, on a host with the recording host's CPU arithmetic:
+    what the unmodified reference returned must come out exactly (reasoning texts and grounding, answers, tokens,
+    detected boxes; every layer's KV cache bit for bit, tests/golden/reference_bitwise.json), and the oracle's own
+    recorded margins, logits and probes within the host-to-host accumulation-order spread (tests/neartie.py)."""
+    from moondream_b200 import config as C, synth
+    from neartie import MARGIN_ULPS_TOL, json_close, reference_bitwise
     from oracle import reference_shim as R
+    from oracle.make_golden_r2 import _grounding_from
+    from oracle.moondream_oracle import OracleModel
 
-    if not R.reference_available():
-        pytest.skip("/root/reference is not on this box")
-    import oracle.make_golden_r2 as G
-
-    G.main(str(tmp_path))                     # asserts oracle == reference on every case while writing
+    kv_sha = reference_bitwise(exact_bf16=True)["round2_kv_sha256"]
+    cfg, sd = tiny
+    tk = cfg.tokenizer
+    stub = R.StubTokenizer(cfg.text.vocab_size)
 
     def tol(path):
         if path.endswith("ulps"):
@@ -135,12 +137,66 @@ def test_round2_restatements_are_bit_identical_to_the_reference_here(tmp_path):
             return 0.25                       # 2 bf16 ulps at |logit| <= 16
         return 2e-3                           # KV probes (means of |k|)
 
-    for n in ("tiny_reasoning.json", "tiny_text_only.json", "tiny_gqa.json", "top_p.json", "tiny_lora.json"):
-        new, old = json.load(open(tmp_path / n)), _gold(n)
-        if n == "top_p.json":                 # the kept sets follow from the logits, which are the host's: compare the inputs
-            for doc in (new, old):
-                for c in doc["cases"]:
-                    for k in ("kept_ids", "kept_probs", "n_kept_by_mass", "mass_before_last_kept", "mass_before_first_dropped"):
-                        c.pop(k)
-        bad = json_close(new, old, tol)
-        assert not bad, f"{n} is stale (commit the regenerated fixture): {bad[:5]}"
+    def close(got, case, what):
+        bad = json_close(got, {k: case[k] for k in got}, tol)
+        assert not bad, (what, bad[:5])
+
+    def kv(enc):
+        return R.tensor_sha256(*[t for pair in enc.caches for t in pair])
+
+    def probe(enc, last):
+        return [float(enc.caches[i][0].float().abs().mean()) for i in (0, last)]
+
+    def reasoning(orc, enc, prompt, max_tokens):
+        r = orc.generate_reasoning(enc, prompt, max_tokens)
+        ans = orc.generate(None, tk.templates["query"]["suffix"], max_tokens, pos=r["pos"])
+        return r, ans, {"reasoning_tokens": r["tokens"], "coords": r["coords"], "margin_ulps": r["margin_ulps"],
+                        "coord_ulps": r["coord_ulps"], "end_margin_ulps": r["end_margin_ulps"],
+                        "answer_tokens": ans.tokens, "answer_margin_ulps": ans.margin_ulps}
+
+    gold = _gold("tiny_reasoning.json")
+    sd_r = dict(sd)
+    sd_r["text.lm_head.bias"] = synth.special_token_bias(sd, cfg, *gold["bias"])
+    orc_r = OracleModel(cfg, sd_r)
+    for c in gold["cases"]:
+        enc = orc_r.encode_image(synth.synthetic_image(c["image_index"], c["height"], c["width"]))
+        r, ans, got = reasoning(orc_r, enc, c["prompt"], c["max_tokens"])
+        assert _grounding_from(r["tokens"], r["coords"], tk, stub.decode) == (c["reasoning_text"], c["grounding"])
+        assert ans.tokens == R.tokens_from_text(c["answer"])
+        close(got, c, "reasoning")
+
+    gold = _gold("tiny_text_only.json")
+    orc = OracleModel(cfg, sd)
+    for c in gold["cases"]:
+        gen = orc.generate(None, c["prompt"], c["max_tokens"])
+        close({"tokens": gen.tokens, "margin_ulps": gen.margin_ulps}, c, "text-only")
+    c = gold["reasoning"]
+    close(reasoning(orc_r, None, c["prompt"], c["max_tokens"])[2], c, "text-only reasoning")
+
+    gcfg = C.tiny_gqa()
+    gorc = OracleModel(gcfg, synth.synthetic_state_dict(gcfg, 0))
+    for c, want in zip(_gold("tiny_gqa.json")["cases"], kv_sha["tiny_gqa"]):
+        enc = gorc.encode_image(synth.synthetic_image(c["image_index"], c["height"], c["width"]))
+        assert kv(enc) == want
+        gen = gorc.generate(enc, c["prompt"], len(c["tokens"]))
+        close({"tokens": gen.tokens, "margin_ulps": gen.margin_ulps,
+               "kv_abs_mean_first_last": probe(enc, gcfg.text.n_layers - 1)}, c, "gqa")
+
+    gold = _gold("tiny_lora.json")
+    orc.lora = synth.nest_lora(synth.synthetic_lora(cfg, gold["rank"], gold["seed"]))
+    for c, want in zip(gold["cases"], kv_sha["tiny_lora"]):
+        enc = orc.encode_image(synth.synthetic_image(c["image_index"], c["height"], c["width"]))
+        assert kv(enc) == want
+        gen = orc.generate(enc, c["prompt"], len(c["tokens"]))
+        det = orc.generate_points(enc, c["detect_prompt"], True, 2)
+        assert len(det) == len(c["detect_boxes"]) and [{k: o[k] for k in d} for o, d in zip(det, c["detect_boxes"])] == c["detect_boxes"]
+        close({"tokens": gen.tokens, "margin_ulps": gen.margin_ulps, "detect_bins": [o["bins"] for o in det],
+               "detect_ulps": [o["ulps"] for o in det], "kv_abs_mean_first_last": probe(enc, cfg.text.n_layers - 1)},
+              c, "lora")
+    orc.lora = None
+
+    # _apply_top_p's inputs: the oracle's prefill logits on image 0 (its kept sets are test_apply_top_p_matches_the_reference)
+    enc = orc.encode_image(synth.synthetic_image(0, 378, 378))
+    for c in _gold("top_p.json")["cases"]:
+        orc.load_encoded(enc)
+        close({"logits": orc.prefill_prompt(c["prompt"], enc.pos)[0][0].float().tolist()}, c, "top_p")

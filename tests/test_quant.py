@@ -101,22 +101,18 @@ def test_int4_dequantisation_matches_the_reference_vectors():
 
 
 def test_int4_against_the_reference_function_when_present():
-    from oracle import reference_shim as R
+    """against dequantize_tensor of the unmodified reference (layers.py:38-44, tests/golden/reference_bitwise.json)"""
+    from neartie import reference_bitwise
 
-    if not R.reference_available():
-        pytest.skip("reference not present (GPU box)")
-    import sys
-
-    sys.path.insert(0, R.REFERENCE_ROOT)
-    from moondream.torch.layers import dequantize_tensor as ref
-
+    from oracle.make_golden_bitwise import INT4_CASES
     from oracle.make_golden_quant import make_case
+    from oracle.reference_shim import tensor_sha256
 
-    for seed, (o, i, awk) in enumerate([(32, 384, True), (128, 128, False), (6, 2048, True)]):
+    gold = reference_bitwise()["int4_dequant"]
+    assert len(gold) == len(INT4_CASES) == 3
+    for seed, ((o, i, awk), want) in enumerate(zip(INT4_CASES, gold)):
         nib, scale, zero = make_case(100 + seed, o, i, awk)
-        packed = quant.pack_reference_int4(nib)
-        want = ref(packed.clone(), scale.reshape(-1, 1), zero.reshape(-1, 1), (o, i), torch.bfloat16)
-        assert torch.equal(want, quant.dequantize(nib, scale, zero))
+        assert tensor_sha256(quant.dequantize(nib, scale, zero)) == want
 
 
 def test_int4_layout_round_trips_and_error_bound():
